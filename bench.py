@@ -13,9 +13,13 @@ lasermap_fov_segment -> update_iterated_dyn_share_modified (h_share_model 5-NN +
 Prints ONE JSON line (rank 0).  PyTorch is used only for pinned/device buffers, stream events and the NCCL barrier.
 
 Frame schedule (identical for both arms, independent of --steps): the workload is N_SCANS scans generated once from the
-seed; frames 0..PARITY_FRAMES-1 are replayed first, in order, from the freshly built map (the GPU posteriors of these
-frames are compared with the CPU replay of the same frames: the `parity` key); the timed K-step blocks follow in frame
-order; when the scan list is used up the map is rebuilt (untimed) and the next cycle starts with W warm-up frames.
+seed; frames 0..max(PARITY_FRAMES, W)-1 are replayed first, in order, from the freshly built map (the GPU posteriors of
+frames 0..PARITY_FRAMES-1 are compared with the CPU replay of the same frames: the `parity` key); the K timed steps follow
+in frame order (wrapping around the scan list when K is larger).  The other timed rows (e2e, sequential) each start from
+a rebuilt map (untimed) with W warm-up frames and time K steps too.
+
+  --dump-outputs DIR   after the timed steps, write what the last timed step computed (posterior state, covariance,
+                       counters, the map it left) as DIR/<name>.npy, for output-for-output comparison of two builds
 """
 import argparse
 import json
@@ -38,7 +42,8 @@ MAP_AREA = 112000.0  # bounding area (m^2) of the pre-filled region that yields 
 N_SCANS = 120        # scans of the cfg2 workload (fixed: map extent and RNG stream do not depend on --steps)
 PARITY_FRAMES = 25   # frames replayed first (GPU and CPU) for the per-frame pose parity
 REF_STEPS_CAP = 12   # --impl reference: bounded sample (~0.35 s of CPU work per step)
-MIN_TIMED_MS = 500.0  # the K-step block is repeated until this much device time has been measured
+MIN_TIMED_MS = 500.0  # a timed window shorter than this is noted on stderr (more --steps give a steadier figure)
+DUMP_BYTES = 64 << 20  # --dump-outputs: at most this much in all
 SEED = 20
 
 
@@ -123,8 +128,9 @@ def workload_config():
     return {"workload": "cfg2: HDL-64 120k-ray scans (Q-raw), 0.2 m voxel, ~5M-pt map, max_iteration=3; one independent "
                         "session per GPU (cfg5: the same route and map on every GPU = fixed per-GPU work, own range noise and priors)",
             "seed": SEED, "n_scans": n_scans_default(), "parity_frames": parity_frames_default(),
-            "frame_schedule": "cycle 0: frames 0..parity_frames-1 from the fresh map (untimed, checked against the CPU replay), "
-                              "then blocks of K consecutive frames; later cycles: map rebuilt (untimed), W warm-up frames, blocks of K",
+            "frame_schedule": "cycle 0: frames 0..max(parity_frames, W)-1 from the fresh map (untimed, frames 0..parity_frames-1 "
+                              "checked against the CPU replay), then K consecutive timed frames; every further timed row: map "
+                              "rebuilt (untimed), W warm-up frames, K frames",
             "pipeline": "replay: two steps in flight",
             "l2_policy": "inputs larger than L2: ~480 MB of map block storage + a new 1.9 MB scan every step",
             "reference_arm": f"same workload and frame schedule; steps capped at {REF_STEPS_CAP} (bounded CPU sample)"}
@@ -273,11 +279,31 @@ def aggregate_scans_per_s(world_size, steps, ms_max):
     return world_size * steps / (ms_max * 1e-3)
 
 
-def block_plan(first_block_ms, min_total_ms=MIN_TIMED_MS, lo=5, hi=400):
-    """How many K-step blocks to time so that >= min_total_ms of device time is measured (at least `lo`, at most `hi`)."""
-    if not (first_block_ms > 0):
-        return lo
-    return int(min(hi, max(lo, np.ceil(min_total_ms / first_block_ms))))
+def map_sample(pts, max_rows):
+    """The map's points in sorted row order; above max_rows, the points whose coordinate hash falls below a fixed
+    threshold (a sample that depends on each point alone, so two nearly equal maps give nearly equal samples)."""
+    pts = np.ascontiguousarray(pts, np.float32)
+    if len(pts) > max_rows:
+        b = pts.view(np.uint32).astype(np.uint64)
+        h = (b[:, 0] * 73856093 ^ b[:, 1] * 19349663 ^ b[:, 2] * 83492791) & 0xFFFFFFFF
+        pts = pts[h < np.uint64(int(0.95 * max_rows / len(pts) * 2 ** 32))]
+    return pts[np.lexsort((pts[:, 2], pts[:, 1], pts[:, 0]))][:max_rows]
+
+
+def dump_outputs(out_dir, state, P, r, map_points):
+    """What the last timed step handed its caller: posterior state (x26) and covariance (23x23), the step's counters
+    (update passes, search passes, effective features, converged count, total residual, points added with / without
+    downsampling, points deleted, map size; timings left out) and the map it left (float32 xyz rows, sorted)."""
+    os.makedirs(out_dir, exist_ok=True)
+    u = r.update
+    counters = np.array([u.passes, u.search_passes, u.effct_feat_num, u.converged_count, u.total_residual, r.n_to_add,
+                         r.n_no_downsample, r.n_deleted, r.map_valid], np.float64)
+    arrays = {"state": np.asarray(state, np.float64), "covariance": np.asarray(P, np.float64), "counters": counters}
+    room = DUMP_BYTES - sum(a.nbytes for a in arrays.values()) - 4096
+    arrays["map_points"] = map_sample(map_points, room // 12)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    log(f"dumped {', '.join(f'{k}{list(v.shape)}' for k, v in arrays.items())} to {out_dir}")
 
 
 def quat_angle(qa, qb):
@@ -387,21 +413,18 @@ def run_b200(args):
         torch.cuda.synchronize()
 
     # ---------------- frame schedule.  A CYCLE starts from the freshly built map: `w` untimed frames 0..w-1 (cycle 0:
-    # w = F, their posteriors are the ones checked against the CPU replay — the `parity` key; later cycles: w = W warm-up
-    # steps), then as many blocks of exactly K consecutive frames as fit into the scan list.  The map is rebuilt (untimed)
-    # between cycles so that every timed block sees the same, well-defined map state: replaying a scan list over and over
-    # into ONE map would keep appending its verbatim (PointNoNeedDownsample) points and grow overflow chains no real
-    # trajectory produces.
+    # w = max(F, W), the posteriors of frames 0..F-1 are the ones checked against the CPU replay — the `parity` key; later
+    # cycles: w = W warm-up steps), then one block of exactly K consecutive frames.  The map is rebuilt (untimed) between
+    # cycles so that every timed block sees the same, well-defined map state: replaying a scan list over and over into ONE
+    # map would keep appending its verbatim (PointNoNeedDownsample) points and grow overflow chains no real trajectory
+    # produces.  Nothing in the schedule depends on a measured time, so the same arguments replay the same frames.
     fov_box = [fov]
 
-    def cycle_blocks(w):
-        starts = list(range(w, NS - K + 1, K)) or [w]
-        if NCU_SHORT:
-            starts = starts[:1]
-        return [[(s0 + j) % NS for j in range(K)] for s0 in starts]
+    def block(w):
+        return [(w + j) % NS for j in range(K)]
 
     def begin_cycle(first):
-        w = F if first else max(W, 0)
+        w = max(F, W) if first else max(W, 0)
         if not first:
             build_map(tree, work["map"])
             fov_box[0] = capi.make_fov(cube_len=1000.0, det_range=100.0)
@@ -422,12 +445,11 @@ def run_b200(args):
     clocks.wait_first()
     barrier()
     w0, settle = begin_cycle(True)
-    post = [st for _, st in settle]
-    valid_after = settle[-1][0].map_valid if settle else 0
+    post = [st for _, st in settle[:F]]
+    valid_after = settle[F - 1][0].map_valid if settle else 0
 
     # ---------------- timed region 1: inputs resident in HBM (value).  One block = EXACTLY K steps between a barrier +
-    # synchronize on both sides, timed with CUDA events on the library stream; blocks are repeated (over as many cycles as
-    # needed) until >= 0.5 s of device time has been measured and the MEDIAN block (of the max over ranks) is reported.
+    # synchronize on both sides, timed with CUDA events on the library stream (max over ranks).
     def timed_block(idx, pipelined=True):
         # the harness keeps its own work out of the timed loop (a C++ caller has none): states/covariances are staged
         # beforehand, results are inspected afterwards
@@ -456,7 +478,7 @@ def run_b200(args):
         e1.record(stream)
         barrier()
         perr = max(float(np.linalg.norm(sts[j][:3] - work["truths"][idx[j]][:3])) for j in range(K))
-        return e0.elapsed_time(e1), sum(r.kernel_launches for r in res), sum(nk_all[k] for k in idx), perr
+        return e0.elapsed_time(e1), sum(r.kernel_launches for r in res), sum(nk_all[k] for k in idx), perr, (sts[-1], Ps[-1], res[-1])
 
     # ---------------- timed region 2: host buffers through the C ABI (e2e).  Streaming use of the public API: every
     # step's scan is copied from pinned host memory inside the region (flb_scan_prefetch, overlapping the previous
@@ -501,44 +523,25 @@ def run_b200(args):
         return dt * 1e3, lat, sum(r.update.passes for r in res2), sum(nk_all[k] for k in idx)
 
     row_lo = clocks.mark()
-    blocks = [timed_block(idx) for idx in cycle_blocks(w0)]            # cycle 0: the blocks after the parity frames
-    blocks_per_cycle = [len(blocks)]
-    first_ms = dist_max([float(np.median([b[0] for b in blocks]))], device=devname)[0]
-    nblocks = block_plan(first_ms) if not (TINY or NCU_SHORT) else (2 if TINY else 1)
-    while len(blocks) < nblocks:
-        w, _ = begin_cycle(False)
-        n0 = len(blocks)
-        for idx in cycle_blocks(w):
-            blocks.append(timed_block(idx))
-        blocks_per_cycle.append(len(blocks) - n0)
+    own_ms, launches, npts, perr, last = timed_block(block(w0))
     row_hi = clocks.mark()
-    ms_blocks = np.array(dist_max([b[0] for b in blocks], device=devname))   # per block: max over ranks
-    order = np.argsort(ms_blocks)
-    bmed = int(order[len(order) // 2])
-    ms = float(ms_blocks[bmed])
-    launches, npts, perr = blocks[bmed][1], blocks[bmed][2], max(b[3] for b in blocks)
-    eblocks = []
-    while len(eblocks) < (min(nblocks, 60) if not (TINY or NCU_SHORT) else (2 if TINY else 1)):
-        w, _ = begin_cycle(False)
-        for idx in cycle_blocks(w):
-            eblocks.append(e2e_block(idx))
-    e2e_ms_blocks = np.array(dist_max([b[0] for b in eblocks], device=devname))
-    e2e_ms = float(np.median(e2e_ms_blocks))
-    lat = np.concatenate([b[1] for b in eblocks])
-    passes = sum(b[2] for b in eblocks) / len(eblocks)
-    # the strictly alternating begin / finish figures (a live filter, whose next prior needs this posterior), one cycle each
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *last, tree.flatten())
+    ms = dist_max([own_ms], device=devname)[0]
+    if ms < MIN_TIMED_MS and not (TINY or NCU_SHORT):
+        log(f"note: the {K} timed steps took {ms:.1f} ms of device time; more --steps give a steadier figure")
     w, _ = begin_cycle(False)
-    seq_blocks = [timed_block(idx, pipelined=False) for idx in cycle_blocks(w)]
+    own_e2e_ms, lat, passes, _ = e2e_block(block(w))
+    e2e_ms = dist_max([own_e2e_ms], device=devname)[0]
+    # the strictly alternating begin / finish figures (a live filter, whose next prior needs this posterior)
     w, _ = begin_cycle(False)
-    seq_eblocks = [e2e_block(idx, pipelined=False) for idx in cycle_blocks(w)]
-    seq_ms = float(np.median(dist_max([b[0] for b in seq_blocks], device=devname)))
-    seq_e2e_ms = float(np.median(dist_max([b[0] for b in seq_eblocks], device=devname)))
-    seq_lat = np.concatenate([b[1] for b in seq_eblocks])
+    seq_ms = dist_max([timed_block(block(w), pipelined=False)[0]], device=devname)[0]
+    w, _ = begin_cycle(False)
+    seq_e2e_ms, seq_lat, _, _ = e2e_block(block(w), pipelined=False)
+    seq_e2e_ms = dist_max([seq_e2e_ms], device=devname)[0]
     clk = clocks.stop(row_lo, row_hi)
-    # per-rank view of the same measurement: own median block time, own GPU's clocks, own e2e
-    mine = [float(np.median([b[0] for b in blocks])), float(np.min([b[0] for b in blocks])), float(np.max([b[0] for b in blocks])),
-            float(np.median([b[0] for b in eblocks])), float(clk["sm_mhz"] or 0.0), float(clk["sm_max_mhz"] or 0.0),
-            float(len(clk["reasons"]))]
+    # per-rank view of the same measurement: own block time, own GPU's clocks, own e2e
+    mine = [own_ms, own_e2e_ms, float(clk["sm_mhz"] or 0.0), float(clk["sm_max_mhz"] or 0.0), float(len(clk["reasons"]))]
     per_rank = dist_gather(mine, device=devname)
     fov = fov_box[0]
 
@@ -578,24 +581,18 @@ def run_b200(args):
             "config": workload_config(),
             "workload_stats": {"scan_points_mean": n_mean, "map_valid": int(stats["valid_points"]),
                                "map_block_storage_mb": stats["blocks_in_use"] * 1024 / 1e6, "pose_err_vs_truth_max_m": perr},
-            "timing": {"what": f"{len(blocks)} blocks of exactly {K} steps, each between barrier+synchronize, CUDA events on the "
-                               "library stream, max over ranks per block; value = median block",
+            "timing": {"what": f"one block of exactly {K} steps (frames {w0}..{w0 + K - 1} mod {NS}) between barrier+synchronize, "
+                               "CUDA events on the library stream, max over ranks",
                        "pipeline": "two steps in flight (flb_scan_step_begin of scan j+1 before flb_scan_step_finish of scan j: replay, the "
                                    "priors are known); `sequential` = strictly alternating begin / finish",
                        "sequential": {"value": aggregate_scans_per_s(world_size, K, seq_ms), "e2e": aggregate_scans_per_s(world_size, K, seq_e2e_ms),
-                                      "blocks": len(seq_blocks), "latency_ms_p50": float(np.percentile(seq_lat, 50) * 1e3),
+                                      "latency_ms_p50": float(np.percentile(seq_lat, 50) * 1e3),
                                       "latency_ms_p99": float(np.percentile(seq_lat, 99) * 1e3)},
-                       "blocks": len(blocks), "block_ms_median": ms, "block_ms_min": float(ms_blocks.min()),
-                       "block_ms_max": float(ms_blocks.max()), "device_ms_total": float(ms_blocks.sum()),
-                       "block_ms": [round(float(x), 4) for x in ms_blocks], "blocks_per_cycle": blocks_per_cycle,
-                       "value_min": aggregate_scans_per_s(world_size, K, float(ms_blocks.max())),
-                       "value_max": aggregate_scans_per_s(world_size, K, float(ms_blocks.min())),
-                       "e2e_blocks": len(eblocks), "e2e_block_ms_min": float(e2e_ms_blocks.min()),
-                       "e2e_block_ms_max": float(e2e_ms_blocks.max())},
-            "per_rank": [{"rank": i, "block_ms_median": r[0], "block_ms_min": r[1], "block_ms_max": r[2], "e2e_block_ms_median": r[3],
-                          "sm_mhz": r[4], "sm_max_mhz": r[5], "throttle_reasons": int(r[6])} for i, r in enumerate(per_rank)],
+                       "block_ms": ms, "e2e_block_ms": e2e_ms},
+            "per_rank": [{"rank": i, "block_ms": r[0], "e2e_block_ms": r[1], "sm_mhz": r[2], "sm_max_mhz": r[3],
+                          "throttle_reasons": int(r[4])} for i, r in enumerate(per_rank)],
             "slowest_rank": int(np.argmax([r[0] for r in per_rank])),
-            "sum_of_rank_rates": float(sum(K / (r[0] * 1e-3) for r in per_rank)),   # (each rank's own median block; NOT the headline)
+            "sum_of_rank_rates": float(sum(K / (r[0] * 1e-3) for r in per_rank)),   # (each rank's own block; NOT the headline)
             "gpu_launches": launches,
             "latency_ms": {"p50": float(np.percentile(lat, 50) * 1e3), "p99": float(np.percentile(lat, 99) * 1e3),
                            "max": float(lat.max() * 1e3), "samples": int(len(lat)),
@@ -816,6 +813,8 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--ncu-short", action="store_true", help="profiling runs under ncu: 3 settle frames, one timed block, no extra rows")
     ap.add_argument("--tiny", action="store_true", help="test-only: shrink the workload (not a bench configuration)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed as DIR/<name>.npy (state, covariance, counters, map)")
     args = ap.parse_args()
     global TINY, NCU_SHORT
     TINY = args.tiny

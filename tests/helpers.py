@@ -1,4 +1,8 @@
 """Shared scene builders for the parity tests (seeded, small enough for the CPU oracle to finish in seconds)."""
+import hashlib
+import json
+import os
+
 import numpy as np
 
 from better_fastlio2_b200 import synth
@@ -113,3 +117,121 @@ def map_properties(tree, queries, rng, n_brute=32):
         for j in range(len(near)):
             assert np.array_equal(brute_knn_d2(after, near[j]), d3[j][:c3[j]])
     return dict(map_points=len(content), queries=len(queries), deleted=nd)
+
+
+# ---------------------------------------------------------------------------------------------- recorded reference ikd-Tree
+# The reference's own ikd-Tree is compiled (oracle/_ref) only where its source is present.  What it returned on the call
+# sequences of the tests that compare a map with it is kept in tests/golden/ref_ikdtree.json (tests/golden/make_golden_ref.py),
+# so those tests run everywhere: the map under test goes through the same calls and must return the same results.
+REF_GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ref_ikdtree.json")
+
+
+def digest(*arrays):
+    h = hashlib.sha256()
+    for a in arrays:
+        a = np.ascontiguousarray(a)
+        h.update(f"{a.dtype.str}{a.shape}".encode())
+        h.update(a.tobytes())
+    return h.hexdigest()[:32]
+
+
+def knn_digest(d2, pts, cnt):
+    """What knn_equal compares, as one digest: counts, which distances are finite, the finite distances bit for bit and the
+    neighbour records (xyz, or xyz + intensity) of every query without a tied distance."""
+    fin = np.isfinite(d2)
+    tie = np.zeros(len(d2), bool)
+    for j in range(d2.shape[1] - 1):
+        tie |= (d2[:, j] == d2[:, j + 1]) & fin[:, j]
+    p = pts[~tie]
+    return digest(np.asarray(cnt, np.int32), fin, d2[fin], np.where(np.isfinite(p), p, 0).astype(p.dtype))
+
+
+def _rows4(a):
+    a = np.ascontiguousarray(a, np.float32)
+    return a[np.lexsort((a[:, 3], a[:, 2], a[:, 1], a[:, 0]))]
+
+
+class RecordedMap:
+    """A map back end (reference ikd-Tree, oracle port or the GPU map) that logs every call as [name, digest of the inputs,
+    result]: counts as they are, k-NN results as knn_digest, point sets as the digest of their sorted rows."""
+
+    def __init__(self, tree):
+        self.tree, self.calls = tree, []
+
+    def _log(self, name, inputs, result=None):
+        self.calls.append([name, digest(*[np.asarray(a) for a in inputs]), result])
+
+    def Build(self, pts):
+        self.tree.Build(pts)
+        self._log("Build", [pts])
+
+    def Build_xyzi(self, pts4):
+        self.tree.Build_xyzi(pts4)
+        self._log("Build_xyzi", [pts4])
+
+    def Add_Points(self, pts, downsample_on):
+        n = int(self.tree.Add_Points(pts, downsample_on))
+        self._log("Add_Points", [pts, downsample_on], n)
+        return n
+
+    def Add_Points_xyzi(self, pts4, downsample_on):
+        n = int(self.tree.Add_Points_xyzi(pts4, downsample_on))
+        self._log("Add_Points_xyzi", [pts4, downsample_on], n)
+        return n
+
+    def Delete_Point_Boxes(self, boxes):
+        n = int(self.tree.Delete_Point_Boxes(boxes))
+        self._log("Delete_Point_Boxes", [boxes], n)
+        return n
+
+    def Delete_Points(self, pts):
+        n = self.tree.Delete_Points(pts)   # the reference returns nothing
+        self._log("Delete_Points", [pts])
+        return n
+
+    def Nearest_Search(self, q, k=5, max_dist=0.0):
+        if not max_dist:
+            out = self.tree.Nearest_Search(q, k)
+        elif hasattr(self.tree, "Nearest_Search_md"):
+            out = self.tree.Nearest_Search_md(q, k, max_dist)
+        else:
+            out = self.tree.Nearest_Search(q, k, max_dist=max_dist)
+        self._log("Nearest_Search", [q, k, max_dist], knn_digest(out[1], out[0], out[2]))
+        return out
+
+    def Nearest_Search_xyzi(self, q, k=5):
+        out = self.tree.Nearest_Search_xyzi(q, k)
+        self._log("Nearest_Search_xyzi", [q, k], knn_digest(out[1], out[0], out[2]))
+        return out
+
+    def flatten(self):
+        a = self.tree.flatten()
+        self._log("flatten", [], digest(sort_rows(a)))
+        return a
+
+    def flatten_xyzi(self):
+        a = self.tree.flatten_xyzi()
+        self._log("flatten_xyzi", [], digest(_rows4(a)))
+        return a
+
+    def validnum(self):
+        n = int(self.tree.validnum())
+        self._log("validnum", [], n)
+        return n
+
+    def close(self):
+        self.tree.close()
+
+
+def assert_matches_reference(rec, case, ignore_results_of=()):
+    """The calls logged in `rec` returned what the reference ikd-Tree returned on the same calls (`case` in REF_GOLDEN).
+    ignore_results_of: calls whose return value is defined differently by the map under test (e.g. the GPU map's Add_Points
+    counts changed voxels, the reference counts sequential add operations); their inputs are still checked."""
+    with open(REF_GOLDEN) as f:
+        want = json.load(f)[case]
+    got = rec.calls
+    for i, (g, w) in enumerate(zip(got, want)):
+        assert g[0] == w[0] and g[1] == w[1], f"{case}: call {i} {g[0]} differs from the recorded call {w[0]} (inputs changed?)"
+        if g[0] not in ignore_results_of:
+            assert g[2] == w[2], f"{case}: call {i} {g[0]} returned {g[2]}, the reference ikd-Tree {w[2]}"
+    assert len(got) == len(want), f"{case}: {len(got)} calls, {len(want)} recorded"
