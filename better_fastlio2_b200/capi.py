@@ -64,6 +64,16 @@ class Profile(C.Structure):
 
 K_CLASSES = ["transform", "knn", "residual", "reduce", "classify", "insert", "delete"]
 
+class PreprocessCfg(C.Structure):
+    _fields_ = [("lidar_type", C.c_int), ("n_scans", C.c_int), ("scan_rate", C.c_int), ("point_filter_num", C.c_int),
+                ("time_unit", C.c_int), ("blind", C.c_double), ("feature_enabled", C.c_int)]
+
+
+class RawLayout(C.Structure):
+    _fields_ = [(k, C.c_int) for k in ("stride", "off_x", "off_y", "off_z", "off_intensity", "off_time", "off_ring", "off_tag",
+                                       "off_line")]
+
+
 _lib = None
 
 # every symbol include/fastlio_b200.h declares
@@ -78,7 +88,7 @@ EXPORTS = [
     "flb_map_profile_enable", "flb_map_profile_read", "flb_session_set_update_engine", "flb_scan_prefetch", "flb_scan_step_begin", "flb_scan_step_finish",
     "flb_frontend_create", "flb_frontend_destroy", "flb_frontend_upload", "flb_frontend_undistort",
     "flb_frontend_voxel_filter", "flb_frontend_process", "flb_frontend_download_undistorted", "flb_frontend_download_down",
-    "flb_frontend_points_to_world", "flb_voxel_grid_filter", "flb_map_reconstruct_keyframes",
+    "flb_frontend_points_to_world", "flb_voxel_grid_filter", "flb_map_reconstruct_keyframes", "flb_frontend_preprocess",
     "flb_map_build_pt", "flb_map_reconstruct_pt", "flb_map_add_points_pt", "flb_map_nearest_search_xyzi",
     "flb_map_box_search_xyzi", "flb_map_radius_search_xyzi", "flb_map_flatten_xyzi", "flb_scan_upload_pt",
 ]
@@ -148,6 +158,8 @@ def lib():
         L.flb_frontend_destroy.argtypes = [vp]
         L.flb_frontend_destroy.restype = None
         L.flb_frontend_upload.argtypes = [vp, vp, C.c_int, C.c_int, C.c_int, C.c_int]
+        L.flb_frontend_preprocess.argtypes = [vp, vp, C.c_int, C.POINTER(RawLayout), C.POINTER(PreprocessCfg), ip,
+                                              C.POINTER(C.c_float)]
         L.flb_frontend_undistort.argtypes = [vp, dp, C.c_int, dp]
         L.flb_frontend_voxel_filter.argtypes = [vp, C.c_float, ip]
         L.flb_frontend_process.argtypes = [vp, vp, C.c_int, C.c_int, C.c_int, C.c_int, dp, C.c_int, dp, C.c_float, ip]
@@ -491,6 +503,29 @@ def pack_pointtype(xyz, intensity=None, curvature=None):
     return buf
 
 
+LIDAR_LIVOX, LIDAR_VELO16, LIDAR_OUST64 = 1, 2, 3   # preprocess.h LID_TYPE
+# The driver records each handler reads (preprocess.h: velodyne_ros::Point, ouster_ros::Point; livox_ros_driver
+# CustomPoint), with the C++ layouts of those structs.
+VELODYNE_RECORD = np.dtype({"names": ["x", "y", "z", "intensity", "time", "ring"],
+                            "formats": ["<f4", "<f4", "<f4", "<f4", "<f4", "<u2"], "offsets": [0, 4, 8, 16, 20, 24], "itemsize": 32})
+OUSTER_RECORD = np.dtype({"names": ["x", "y", "z", "intensity", "t", "reflectivity", "ring", "ambient", "range"],
+                          "formats": ["<f4", "<f4", "<f4", "<f4", "<u4", "<u2", "u1", "<u2", "<u4"],
+                          "offsets": [0, 4, 8, 16, 20, 24, 26, 28, 32], "itemsize": 48})
+LIVOX_RECORD = np.dtype({"names": ["offset_time", "x", "y", "z", "reflectivity", "tag", "line"],
+                         "formats": ["<u4", "<f4", "<f4", "<f4", "u1", "u1", "u1"], "offsets": [0, 4, 8, 12, 16, 17, 18],
+                         "itemsize": 20})
+# field names per lidar type: (intensity, time, ring, tag, line)
+_PP_FIELDS = {LIDAR_VELO16: ("intensity", "time", "ring", None, None), LIDAR_OUST64: ("intensity", "t", None, None, None),
+              LIDAR_LIVOX: ("reflectivity", "offset_time", None, "tag", "line")}
+
+
+def raw_layout(dtype, lidar_type):
+    """flb_raw_layout of a structured dtype, by field name; missing fields are -1."""
+    off = lambda name: dtype.fields[name][1] if name and name in dtype.fields else -1
+    fi, ft, fr, fg, fl = _PP_FIELDS.get(int(lidar_type), (None,) * 5)
+    return RawLayout(dtype.itemsize, off("x"), off("y"), off("z"), off(fi), off(ft), off(fr), off(fg), off(fl))
+
+
 class FrontEnd:
     """Device front end of one session: meas.lidar -> UndistortPcl -> VoxelGrid -> feats_down_body (SURVEY.md §8f)."""
 
@@ -521,6 +556,22 @@ class FrontEnd:
     def upload_ptr(self, ptr, n, stride=POINT_STRIDE, off_i=OFF_INTENSITY, off_c=OFF_CURVATURE):
         _chk(lib().flb_frontend_upload(self.h, C.c_void_p(ptr), int(n), stride, off_i, off_c))
         self.n_raw = int(n)
+
+    def preprocess(self, records, lidar_type, n_scans=16, scan_rate=10, point_filter_num=1, time_unit=2, blind=0.01,
+                   feature_enabled=0, layout=None):
+        """Preprocess::process on the device: records is a numpy structured array of driver records (e.g. VELODYNE_RECORD,
+        OUSTER_RECORD, LIVOX_RECORD); the field layout is taken from its dtype by name unless `layout` is given.
+        Returns (n_out, last_curvature); the front end then holds meas.lidar as after upload()."""
+        rec = np.ascontiguousarray(records)
+        lay = layout if layout is not None else raw_layout(rec.dtype, lidar_type)
+        cfg = PreprocessCfg(int(lidar_type), int(n_scans), int(scan_rate), int(point_filter_num), int(time_unit), float(blind),
+                            int(feature_enabled))
+        n = C.c_int(0)
+        last = C.c_float(0.0)
+        _chk(lib().flb_frontend_preprocess(self.h, rec.ctypes.data if len(rec) else None, len(rec), C.byref(lay), C.byref(cfg),
+                                           C.byref(n), C.byref(last)))
+        self.n_raw = n.value
+        return n.value, last.value
 
     def undistort(self, imu_poses, state26_end):
         poses = np.ascontiguousarray(imu_poses, np.float64).reshape(-1, 22)

@@ -27,7 +27,9 @@ static int vg_ensure(VgWork& w, int n) {
   size_t t1 = 0, t2 = 0;
   CU(cub::DeviceRadixSort::SortPairs(nullptr, t1, (const unsigned*)nullptr, (unsigned*)nullptr, (const int*)nullptr, (int*)nullptr, cap));
   CU(cub::DeviceScan::ExclusiveSum(nullptr, t2, (const int*)nullptr, (int*)nullptr, cap));
-  w.tmp_bytes = std::max(t1, t2) + 256;
+  size_t t3 = 0;   // the segmented chain scan of the Velodyne yaw-time preprocess
+  CU(cub::DeviceScan::InclusiveScan(nullptr, t3, (const unsigned*)nullptr, (unsigned*)nullptr, flb::PpChainOp(), cap));
+  w.tmp_bytes = std::max(std::max(t1, t2), t3) + 256;
   CU(cudaMalloc((void**)&w.keys_a, sizeof(unsigned) * (size_t)cap));
   CU(cudaMalloc((void**)&w.keys_b, sizeof(unsigned) * (size_t)cap));
   CU(cudaMalloc((void**)&w.vals_a, sizeof(int) * (size_t)cap));
@@ -83,6 +85,9 @@ struct flb_frontend {
   cudaEvent_t ev_poses = nullptr;
   VgWork vg;
   bool holds_ref = false;
+  float* pp_t = nullptr;    // preprocess: synthesised Velodyne times by raw index (allocated on first use)
+  int* pp_ring = nullptr;   // preprocess: sorted position of each ring's first point, n_scans + 1 entries
+  int pp_ring_cap = 0;
 };
 
 extern "C" int flb_frontend_create(flb_session* s, int max_raw_points, flb_frontend** out) {
@@ -122,7 +127,7 @@ extern "C" void flb_frontend_destroy(flb_frontend* f) {
   if (!f) return;
   flb_map* m = f->ses ? f->ses->map : nullptr;
   if (m) { Q(cudaSetDevice(m->cfg.device)); Q(cudaStreamSynchronize(m->stream)); }
-  void* ptrs[] = {f->raw, f->pts, f->pts_t, f->world, f->curv, f->curv_t, f->down_curv, f->perm, f->d_poses};
+  void* ptrs[] = {f->raw, f->pts, f->pts_t, f->world, f->curv, f->curv_t, f->down_curv, f->perm, f->d_poses, f->pp_t, f->pp_ring};
   for (void* p : ptrs) if (p) Q(cudaFree(p));
   if (f->h_poses) Q(cudaFreeHost(f->h_poses));
   if (f->ev_poses) Q(cudaEventDestroy(f->ev_poses));
@@ -159,6 +164,141 @@ extern "C" int flb_frontend_upload(flb_frontend* f, const void* pts, int n, int 
   k_pack_xyzic<<<grid_for(n, 256, m->sm_count * 8), 256, 0, m->stream>>>(f->raw, stride, off_intensity, off_curvature, f->pts, f->curv, n);
   m->launches++;
   CU(cudaGetLastError());
+  return 0;
+}
+
+// ------------------------------------------------------------------------------------------------ preprocess
+static int pp_check_field(int off, int size, int stride, const char* name) {
+  if (off < 0) return 0;
+  if (off + size > stride) return set_err("flb_frontend_preprocess: field %s at byte %d lies outside the %d-byte record", name, off, stride);
+  if (off % size) return set_err("flb_frontend_preprocess: field %s at byte %d is not %d-byte aligned", name, off, size);
+  return 0;
+}
+
+extern "C" int flb_frontend_preprocess(flb_frontend* f, const void* records, int n, const flb_raw_layout* layout,
+                                       const flb_preprocess_cfg* cfg, int* n_out, float* last_curvature) {
+  if (!f || !layout || !cfg) return set_err("flb_frontend_preprocess: null argument");
+  if (n < 0 || n > f->cap) return set_err("raw scan of %d points exceeds max_raw_points=%d", n, f->cap);
+  if (n > 0 && !records) return set_err("flb_frontend_preprocess: null records");
+  const int lt = cfg->lidar_type;
+  if (lt != FLB_LIDAR_LIVOX && lt != FLB_LIDAR_VELO16 && lt != FLB_LIDAR_OUST64)
+    return set_err("flb_frontend_preprocess: unsupported lidar_type %d (1 LIVOX, 2 VELO16, 3 OUST64)", lt);
+  if (cfg->feature_enabled) return set_err("flb_frontend_preprocess: feature extraction (feature_enabled) is not supported");
+  if (cfg->point_filter_num < 1) return set_err("point_filter_num must be >= 1 (got %d)", cfg->point_filter_num);
+  if (cfg->n_scans < 1 || cfg->n_scans > 65535) return set_err("n_scans must be in [1, 65535] (got %d)", cfg->n_scans);
+  if (lt == FLB_LIDAR_VELO16 && cfg->scan_rate < 1) return set_err("scan_rate must be >= 1 (got %d)", cfg->scan_rate);
+  const flb_raw_layout& L = *layout;
+  if (L.stride < 1) return set_err("flb_frontend_preprocess: bad record stride %d", L.stride);
+  if (L.off_x < 0 || L.off_y < 0 || L.off_z < 0) return set_err("flb_frontend_preprocess: the x, y and z fields are required");
+  const bool livox = lt == FLB_LIDAR_LIVOX;
+  if (pp_check_field(L.off_x, 4, L.stride, "x") || pp_check_field(L.off_y, 4, L.stride, "y") || pp_check_field(L.off_z, 4, L.stride, "z") ||
+      pp_check_field(L.off_intensity, livox ? 1 : 4, L.stride, livox ? "reflectivity" : "intensity") ||
+      pp_check_field(L.off_time, 4, L.stride, livox ? "offset_time" : "time") ||
+      (lt == FLB_LIDAR_VELO16 && pp_check_field(L.off_ring, 2, L.stride, "ring")) ||
+      (livox && (pp_check_field(L.off_tag, 1, L.stride, "tag") || pp_check_field(L.off_line, 1, L.stride, "line"))))
+    return 1;
+  if (L.stride % 4) return set_err("flb_frontend_preprocess: record stride %d is not a multiple of 4", L.stride);
+  flb_map* m = f->ses->map;
+  CU(cudaSetDevice(m->cfg.device));
+  f->n_raw = 0;
+  f->sorted = false;
+  f->n_down = -1;
+  if (n_out) *n_out = 0;
+  if (last_curvature) *last_curvature = 0.f;
+  // velodyne_handler returns at once on an empty cloud; the others produce nothing from it either
+  if (n == 0) return 0;
+  cudaStream_t st = m->stream;
+  const size_t bytes = (size_t)n * L.stride;
+  if (bytes > f->raw_cap) {
+    if (f->raw) Q(cudaFree(f->raw));
+    f->raw = nullptr; f->raw_cap = 0;
+    const size_t cap = std::max(bytes, (size_t)f->cap * (size_t)L.stride);
+    CU(cudaMalloc((void**)&f->raw, cap));
+    f->raw_cap = cap;
+  }
+  CU(cudaMemcpyAsync(f->raw, records, bytes, cudaMemcpyHostToDevice, st));
+
+  PpArgs a;
+  a.rec = f->raw;
+  a.stride = L.stride; a.off_x = L.off_x; a.off_y = L.off_y; a.off_z = L.off_z; a.off_i = L.off_intensity; a.off_t = L.off_time;
+  a.off_ring = L.off_ring; a.off_tag = L.off_tag; a.off_line = L.off_line;
+  a.n = n; a.n_scans = cfg->n_scans; a.pfn = cfg->point_filter_num;
+  const int tu = cfg->time_unit;
+  a.time_scale = tu == 0 ? 1.e3f : tu == 1 ? 1.f : tu == 2 ? 1.e-3f : tu == 3 ? 1.e-6f : 1.f;
+  a.blind2 = cfg->blind * cfg->blind;
+  a.omega = 0.361 * cfg->scan_rate;
+  int mode = lt == FLB_LIDAR_OUST64 ? PP_OUSTER : livox ? PP_LIVOX : PP_VELO_TIME;
+  if (mode == PP_VELO_TIME) {   // given_offset_time is decided by the last point (:322)
+    float t_last = 0.f;
+    if (L.off_time >= 0) memcpy(&t_last, (const unsigned char*)records + (size_t)(n - 1) * L.stride + L.off_time, sizeof(float));
+    if (!(t_last > 0.f)) mode = PP_VELO_YAW;
+  }
+
+  VgWork& w = f->vg;
+  const int g = grid_for(n, 256, m->sm_count * 8);
+  int* keep = w.flags;
+  int* pos = w.pos;
+  k_vg_init<<<1, 32, 0, st>>>(w.d_mm);   // d_mm[2] = first raw index with ring >= n_scans (none: 0xFFFFFFFF)
+  m->launches++;
+  size_t tb = w.tmp_bytes;
+  if (mode == PP_VELO_YAW) {
+    if (!f->pp_t) CU(cudaMalloc((void**)&f->pp_t, sizeof(float) * (size_t)f->cap));
+    if (cfg->n_scans + 1 > f->pp_ring_cap) {
+      if (f->pp_ring) Q(cudaFree(f->pp_ring));
+      f->pp_ring = nullptr; f->pp_ring_cap = 0;
+      CU(cudaMalloc((void**)&f->pp_ring, sizeof(int) * (size_t)(cfg->n_scans + 1)));
+      f->pp_ring_cap = cfg->n_scans + 1;
+    }
+    int bits = 1;
+    while ((1u << bits) <= (unsigned)cfg->n_scans) ++bits;
+    float* c0 = f->curv_t;   // scratch: undistort rewrites it before anything reads it
+    k_pp_ring_keys<<<g, 256, 0, st>>>(a, w.keys_a, w.vals_a, w.d_mm);
+    CU(cub::DeviceRadixSort::SortPairs(w.tmp, tb, (const unsigned*)w.keys_a, w.keys_b, (const int*)w.vals_a, w.vals_b, n, 0, bits, st));
+    k_pp_ring_start<<<g, 256, 0, st>>>(w.keys_b, n, f->pp_ring);
+    k_pp_yaw_c0<<<g, 256, 0, st>>>(a, w.keys_b, w.vals_b, f->pp_ring, c0);
+    k_pp_yaw_codes<<<g, 256, 0, st>>>(w.keys_b, f->pp_ring, c0, n, a.omega, w.keys_a);
+    tb = w.tmp_bytes;
+    CU(cub::DeviceScan::InclusiveScan(w.tmp, tb, (const unsigned*)w.keys_a, (unsigned*)pos, flb::PpChainOp(), n, st));
+    k_pp_yaw_apply<<<g, 256, 0, st>>>(w.vals_b, c0, (const unsigned*)pos, n, a.omega, f->pp_t);
+    k_pp_keep<PP_VELO_YAW><<<g, 256, 0, st>>>(a, f->pp_ring, w.vals_b, keep);
+    m->launches += 6 + 5 + 1;   // + the radix-sort and scan kernels of CUB
+  } else if (mode == PP_LIVOX) {
+    int* valid = (int*)w.keys_a;
+    int* valid_excl = (int*)w.keys_b;
+    k_pp_livox_valid<<<g, 256, 0, st>>>(a, valid);
+    CU(cub::DeviceScan::ExclusiveSum(w.tmp, tb, (const int*)valid, valid_excl, n, st));
+    k_pp_keep<PP_LIVOX><<<g, 256, 0, st>>>(a, valid, valid_excl, keep);
+    m->launches += 2 + 1;
+  } else if (mode == PP_OUSTER) {
+    k_pp_keep<PP_OUSTER><<<g, 256, 0, st>>>(a, nullptr, nullptr, keep);
+    m->launches++;
+  } else {
+    k_pp_keep<PP_VELO_TIME><<<g, 256, 0, st>>>(a, nullptr, nullptr, keep);
+    m->launches++;
+  }
+  tb = w.tmp_bytes;
+  CU(cub::DeviceScan::ExclusiveSum(w.tmp, tb, (const int*)keep, pos, n, st));
+  switch (mode) {
+    case PP_OUSTER: k_pp_scatter<PP_OUSTER><<<g, 256, 0, st>>>(a, keep, pos, nullptr, f->pts, f->curv, w.d_mm); break;
+    case PP_VELO_TIME: k_pp_scatter<PP_VELO_TIME><<<g, 256, 0, st>>>(a, keep, pos, nullptr, f->pts, f->curv, w.d_mm); break;
+    case PP_VELO_YAW: k_pp_scatter<PP_VELO_YAW><<<g, 256, 0, st>>>(a, keep, pos, f->pp_t, f->pts, f->curv, w.d_mm); break;
+    default: k_pp_scatter<PP_LIVOX><<<g, 256, 0, st>>>(a, keep, pos, nullptr, f->pts, f->curv, w.d_mm); break;
+  }
+  k_pp_last<<<1, 1, 0, st>>>(f->curv, w.d_mm);
+  m->launches += 1 + 2;
+  CU(cudaGetLastError());
+  CU(cudaMemcpyAsync(w.h_mm, w.d_mm, sizeof(unsigned) * 8, cudaMemcpyDeviceToHost, st));
+  CU(cudaStreamSynchronize(st));
+  if (mode == PP_VELO_YAW && w.h_mm[2] != 0xFFFFFFFFu) {
+    const unsigned i = w.h_mm[2];
+    unsigned short ring = 0;
+    memcpy(&ring, (const unsigned char*)records + (size_t)i * L.stride + L.off_ring, sizeof(ring));
+    return set_err("flb_frontend_preprocess: point %u has ring %u >= n_scans=%d (times are synthesised per ring)", i, (unsigned)ring,
+                   cfg->n_scans);
+  }
+  f->n_raw = (int)w.h_mm[0];
+  if (n_out) *n_out = f->n_raw;
+  if (last_curvature) memcpy(last_curvature, &w.h_mm[1], sizeof(float));
   return 0;
 }
 

@@ -310,3 +310,68 @@ def raw_scan_with_times(body_xyz, rng, scan_time_ms=100.0, shuffle=True):
     inten = rng.uniform(0, 255, n).astype(np.float32)
     order = rng.permutation(n) if shuffle else np.arange(n)
     return body_xyz[order].astype(np.float32), inten[order], cur[order].astype(np.float32)
+
+
+# ----------------------------------------------------------------------------------------------- driver records
+def sensor_scan(world, model, rng, columns=None, origin=(0.0, 0.0, 1.8), max_range=100.0, min_range=1.0):
+    """Returns of one sweep in the order the driver sends them: for spinning sensors column by column (all rings of
+    one azimuth, then the next; azimuth decreasing, i.e. clockwise as Velodyne and Ouster spin), for Livox in firing
+    order.  `columns` keeps that many azimuth columns spread over the full turn (spinning) or the first that many
+    returns (Livox).  Returns xyz (float32), ring (int) and the azimuth column
+    (spinning) or firing index (Livox) of every return; rays without a hit are dropped."""
+    d = lidar_dirs(model, rng)
+    if model == "hap":
+        if columns is not None:
+            d = d[:columns]
+        ring = np.arange(len(d)) % 6
+        col = np.arange(len(d))
+    else:
+        n_rings = {"vlp16": 16, "hdl64": 64, "os64": 64}[model]
+        d = d.reshape(n_rings, -1, 3)
+        d = d[:, ::-1]
+        if columns is not None:
+            d = d[:, ::max(1, d.shape[1] // columns)][:, :columns]
+        n_cols = d.shape[1]
+        d = d.transpose(1, 0, 2).reshape(-1, 3)            # column-major: rings interleaved
+        ring = np.tile(np.arange(n_rings), n_cols)
+        col = np.repeat(np.arange(n_cols), n_rings)
+    r = raycast(world, origin, d, max_range=max_range, min_range=min_range)
+    ok = np.isfinite(r)
+    xyz = (d[ok] * r[ok, None]).astype(np.float32)
+    return xyz, ring[ok], col[ok]
+
+
+def velodyne_records(xyz, ring, time_s, rng):
+    from .capi import VELODYNE_RECORD
+    rec = np.zeros(len(xyz), VELODYNE_RECORD)
+    rec["x"], rec["y"], rec["z"] = xyz[:, 0], xyz[:, 1], xyz[:, 2]
+    rec["intensity"] = rng.integers(0, 256, len(xyz)).astype(np.float32)
+    rec["time"] = time_s
+    rec["ring"] = ring
+    return rec
+
+
+def ouster_records(xyz, ring, t_int, rng):
+    from .capi import OUSTER_RECORD
+    rec = np.zeros(len(xyz), OUSTER_RECORD)
+    rec["x"], rec["y"], rec["z"] = xyz[:, 0], xyz[:, 1], xyz[:, 2]
+    rec["intensity"] = rng.uniform(0, 3000, len(xyz)).astype(np.float32)
+    rec["t"] = t_int
+    rec["ring"] = ring
+    rec["reflectivity"] = rng.integers(0, 65536, len(xyz))
+    rec["range"] = (np.linalg.norm(xyz, axis=1) * 1000).astype(np.uint32)
+    return rec
+
+
+def livox_records(xyz, line, offset_ns, rng, tag_mix=True):
+    """CustomMsg points; with tag_mix, about 10 % carry a second/third-return or noise tag."""
+    from .capi import LIVOX_RECORD
+    rec = np.zeros(len(xyz), LIVOX_RECORD)
+    rec["x"], rec["y"], rec["z"] = xyz[:, 0], xyz[:, 1], xyz[:, 2]
+    rec["reflectivity"] = rng.integers(0, 256, len(xyz))
+    rec["offset_time"] = offset_ns
+    rec["line"] = line
+    if tag_mix:
+        rec["tag"] = rng.choice(np.array([0x00, 0x10, 0x20, 0x30, 0x01, 0x12, 0x24], np.uint8), len(xyz),
+                                p=[0.6, 0.2, 0.05, 0.05, 0.04, 0.04, 0.02])
+    return rec

@@ -262,6 +262,36 @@ void flb_frontend_destroy(flb_frontend* f);
  * byte offsets of those float fields inside a point, or -1 when absent (treated as 0).  The buffer holds n whole records
  * (n * stride_bytes bytes are copied), as a std::vector<PointType> / pcl::PointCloud does. */
 int flb_frontend_upload(flb_frontend* f, const void* pts, int n, int stride_bytes, int off_intensity, int off_curvature);
+/* Preprocess::process (src/preprocess.cpp), non-feature branch, on the device: the driver's records -> meas.lidar.
+ * Replaces flb_frontend_upload: one copy of n records of layout->stride bytes, then the handler's blind cut,
+ * point_filter_num decimation and per-point time offset (curvature, ms) run on the GPU, in input order.
+ *   FLB_LIDAR_LIVOX  livox_handler (:178-204): CustomMsg points; x,y,z f32, intensity = reflectivity u8, time =
+ *                    offset_time u32 (ns), tag u8, line u8.  Point 0 is never used.
+ *   FLB_LIDAR_VELO16 velodyne_handler (:417-473): x,y,z,intensity f32, time f32, ring u16.  When the last point's time
+ *                    is not > 0 the times are synthesised per ring from the yaw angle (the first point of each ring is
+ *                    dropped) and every ring must be < n_scans.
+ *   FLB_LIDAR_OUST64 oust64_handler (:271-297): x,y,z,intensity f32, time = t u32.
+ * Offsets of absent fields are -1 (read as 0, as fromROSMsg leaves them); x,y,z are required; f32 / u32 fields must be
+ * 4-byte aligned and u16 fields 2-byte aligned inside the record.  *n_out = pl_surf.size() and *last_curvature =
+ * pl_surf.back().curvature (0 for an empty cloud), what sync_packages reads.  Afterwards the front end holds the cloud
+ * as after flb_frontend_upload of it.  feature_enabled (give_feature) is not supported and is rejected. */
+#define FLB_LIDAR_LIVOX 1
+#define FLB_LIDAR_VELO16 2
+#define FLB_LIDAR_OUST64 3
+typedef struct flb_preprocess_cfg {   /* the Preprocess members set at laserMapping.cpp:2034-2041 */
+  int lidar_type;        /* FLB_LIDAR_* (preprocess.h LID_TYPE) */
+  int n_scans;           /* N_SCANS */
+  int scan_rate;         /* SCAN_RATE (Hz), for the synthesised Velodyne times */
+  int point_filter_num;  /* keep every point_filter_num-th point, >= 1 */
+  int time_unit;         /* 0 s, 1 ms, 2 us, 3 ns (preprocess.h TIME_UNIT; any other value scales by 1) */
+  double blind;          /* blind range (m) */
+  int feature_enabled;   /* must be 0 */
+} flb_preprocess_cfg;
+typedef struct flb_raw_layout {   /* byte offsets inside one record of `stride` bytes; -1 = field absent */
+  int stride, off_x, off_y, off_z, off_intensity, off_time, off_ring, off_tag, off_line;
+} flb_raw_layout;
+int flb_frontend_preprocess(flb_frontend* f, const void* records, int n, const flb_raw_layout* layout,
+                            const flb_preprocess_cfg* cfg, int* n_out, float* last_curvature);
 /* ImuProcess::UndistortPcl, the per-point part (IMU_Processing.hpp:243 sort by time, :334-386 backward compensation).
  * imu_poses = n_poses x 22 doubles = the IMUpose vector built by the forward propagation (:260-322, stays on the host
  * with kf.predict); state26_end = imu_state after the last predict (:329).  Result: feats_undistort in time order

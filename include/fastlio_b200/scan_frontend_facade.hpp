@@ -41,6 +41,7 @@ class ScanFrontEnd {
   // meas.lidar -> device (IMU_Processing.hpp:242 "pcl_out = *(meas.lidar)")
   template <class Cloud>
   bool upload(const Cloud& cloud) {
+    ++gen_;
     typedef typename std::remove_reference<decltype(cloud.points[0])>::type P;
     const int n = (int)cloud.points.size();
     const P* p0 = n ? &cloud.points[0] : nullptr;
@@ -53,7 +54,7 @@ class ScanFrontEnd {
   // predict.  When `out` is given it receives the time-sorted compensated cloud (x,y,z,intensity,curvature), i.e. pcl_out.
   template <class Cloud, class PoseVec, class State>
   bool undistort(const Cloud& lidar, const PoseVec& poses, const State& imu_state, Cloud* out = nullptr) {
-    if (!upload(lidar)) return false;
+    if (!on_device(lidar) && !upload(lidar)) return false;
     std::vector<double> pz(poses.size() * FLB_IMU_POSE_DOUBLES);
     for (size_t k = 0; k < poses.size(); ++k) {
       double* o = &pz[k * FLB_IMU_POSE_DOUBLES];
@@ -107,11 +108,27 @@ class ScanFrontEnd {
     return true;
   }
 
+  // Called by PreprocessGpu after it left `cloud` on the device: until the next upload or preprocess, undistort()
+  // of this very cloud (same object, same point storage and size) uses the device copy instead of uploading it.
+  void device_cloud_replaced() { ++gen_; }
+  template <class Cloud>
+  void mark_on_device(const Cloud& cloud) {
+    dev_gen_ = ++gen_;
+    dev_cloud_ = &cloud;
+    dev_points_ = cloud.points.empty() ? nullptr : (const void*)&cloud.points[0];
+    dev_n_ = cloud.points.size();
+  }
+
  private:
   template <class P>
   static void fill(P& p, const float* v, float curvature) {
     p = P();
     p.x = v[0]; p.y = v[1]; p.z = v[2]; p.intensity = v[3]; p.curvature = curvature;
+  }
+  template <class Cloud>
+  bool on_device(const Cloud& c) const {
+    return dev_gen_ == gen_ && dev_cloud_ == (const void*)&c && dev_n_ == c.points.size() &&
+           dev_points_ == (c.points.empty() ? nullptr : (const void*)&c.points[0]);
   }
   static bool ok(int rc, const char* what) {
     if (rc) std::fprintf(stderr, "[fastlio_b200] %s: %s\n", what, flb_last_error());
@@ -119,6 +136,10 @@ class ScanFrontEnd {
   }
   flb_frontend* fe_ = nullptr;
   std::vector<float> xyzi_, curv_;
+  unsigned long long gen_ = 0, dev_gen_ = 0;   // bumped by every upload / preprocess
+  const void* dev_cloud_ = nullptr;
+  const void* dev_points_ = nullptr;
+  size_t dev_n_ = 0;
 };
 
 // pcl::VoxelGrid<PointT> call shape on top of a ScanFrontEnd.  setInputCloud() is accepted for source compatibility: the
